@@ -2,7 +2,7 @@
 """bench.py -- headline measurement of the GPTQ-4bit hot path on B200 (contract: see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model 7b] [--ctx 1920]
-                    [--groupsize 128] [--act-order] [--seq 2048]
+                    [--groupsize 128] [--act-order] [--seq 2048] [--dump-outputs DIR]
 
 One "step" = one decode token of a Llama-shaped stack on random GPTQ tensors of the named architecture (no checkpoints
 exist offline): every layer's rms_norm + q/k/v projections + rope + cache write, attention over ctx cached positions,
@@ -21,6 +21,9 @@ o_proj + residual, rms_norm + gate/up + silu*mul + down + residual, then final n
 
 --impl reference times that CPU restatement (the reference ships no CPU path for q4; BASELINE.md section 3) and loads
 nothing of this repo's native code.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (the logits, float32) to DIR/logits.npy.
+Weights, KV cache and hidden state are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -50,7 +53,10 @@ def parse():
     ap.add_argument("--no-fused-step", action="store_true", help="time the per-op path even where the persistent kernel applies")
     ap.add_argument("--no-per-op", action="store_true", help="skip the per-op comparison rows (large models: saves time)")
     ap.add_argument("--cpu-seconds", type=float, default=8.0, help="CPU sample budget per repetition (reference arm / cpu_baseline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's logits to DIR/logits.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.ctx is None:
         a.ctx = a.seq - 128
     return a
@@ -151,7 +157,7 @@ def cpu_sample(shape, gs, act, seconds_budget, threads):
     threads: an int, or a list of candidate counts -- the fastest is used (an OpenMP team larger than the CPUs the container
     may use spends its time in spin barriers: 128 threads measured 400x slower than 64 on the round-2 box)."""
     from oracle import oracle as O
-    O.build()
+    O.lib()                                         # built by build(): bench.py compiles nothing into the tree
     dims = [(shape.hidden, shape.hidden)] * 4 + [(shape.hidden, shape.inter)] * 2 + [(shape.inter, shape.hidden)]
     tensors = []
     for i, (K, N) in enumerate(dims):
@@ -238,6 +244,18 @@ def cpu_baseline_subprocess(args):
         return {"value": None, "unit": "tok/s", "cores": host_threads(), "kind": "port", "sample": f"failed: {ex!r}"[:200]}
 
 
+def dump_outputs(directory, arrays):
+    """--dump-outputs: each tensor as DIR/<name>.npy in float32 (64 MB at most: the logits of any SHAPES model are far less)."""
+    import numpy as np
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > 64 << 20:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed 64 MB")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 def main():
     args = parse()
@@ -284,6 +302,7 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    torch.manual_seed(0)                                          # the same step inputs in every run (the weights are seeded too)
     hidden0 = (torch.randn((1, 1, shape.hidden), device=dev) * 0.5).half()
     hidden = hidden0.clone()
     past = args.ctx
@@ -305,8 +324,8 @@ def main():
         torch.cuda.current_stream().wait_stream(side); torch.cuda.synchronize()
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g, capture_error_mode="thread_local"):
-            fn()
-        return g
+            out = fn()
+        return g, out
 
     def time_events(fn, n):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -340,8 +359,12 @@ def main():
         # NCCL inside stream capture hung on this stack; the fused all-reduce kernels are plain launches and capture fine
         use_graph = not args.no_graph and (world == 1 or (fused_ar and not args.act_order) or os.environ.get("EXL_BENCH_TP_GRAPH", "0") == "1")
         # (act-order + tensor parallel falls back to NCCL for the MLP; NCCL inside stream capture hung on this stack in round 1)
-        graph = capture(per_op_step) if use_graph else None
-        step_device = graph.replay if graph is not None else per_op_step
+        graph, graph_out = capture(per_op_step) if use_graph else (None, None)
+
+        def replay():
+            graph.replay()
+            return graph_out
+        step_device = replay if graph is not None else per_op_step
         launches_per_step = launches_per_op
         mode = "per-op kernels, " + ("CUDA graph" if graph is not None else "eager")
 
@@ -357,10 +380,12 @@ def main():
     torch.cuda.cudart().cudaProfilerStart()          # no-op unless run under `ncu --profile-from-start off`
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        out = step_device()
     e1.record()
     barrier()
     torch.cuda.cudart().cudaProfilerStop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"logits": out})
     ms = e0.elapsed_time(e1)
     clocks = sampler.result() if rank == 0 else None
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -387,7 +412,7 @@ def main():
         step_e2e()
     barrier()
     t0 = time.perf_counter()
-    n_e2e = max(8, min(args.steps, 64))
+    n_e2e = args.steps
     for _ in range(n_e2e):
         step_e2e()
     barrier()
@@ -435,7 +460,7 @@ def main():
                     ("down (+residual)", down_all, q4_bytes(il, shape.hidden, gs, act=args.act_order, accumulate=True), 1),
                     ("o_proj (+residual)", o_all, q4_bytes(stack.layers[0].o.height, shape.hidden, gs, act=args.act_order, accumulate=True), 1)]
             for name, fn, by, nlaunch in rows:
-                g = capture(fn)
+                g, _ = capture(fn)
                 for _ in range(2): g.replay()
                 us = time_events(g.replay, 8) * 1e3 / nl
                 kern_rows.append({"kernel": name, "launches": nlaunch, "us": round(us, 3), "bytes": by, "GBps": round(by / us / 1e3, 1),
@@ -461,13 +486,13 @@ def main():
     # ------------------------------------------------------------------ comparison rows: per-op path as a graph, torch attention
     extra = {}
     if world == 1 and not args.no_per_op:
-        g = graph if graph is not None else capture(per_op_step)
+        g = graph if graph is not None else capture(per_op_step)[0]
         for _ in range(3): g.replay()
         per_op_ms = time_events(g.replay, 16)
         extra["decode_per_op_graph"] = {"value": round(1000.0 / per_op_ms, 2), "unit": "tok/s", "launches_per_step": int(launches_per_op),
                                         "note": "the per-op kernels model.py drives (q4_attn, decode_attn, q4_attn_2, q4_mlp) + cuBLAS lm_head, CUDA graph"}
         stack.fused_decode_attn = False
-        g2 = capture(per_op_step)
+        g2, _ = capture(per_op_step)
         for _ in range(3): g2.replay()
         extra["decode_torch_attention"] = {"value": round(1000.0 / time_events(g2.replay, 16), 2), "unit": "tok/s",
                                            "note": "same, with the reference's torch attention ops instead of decode_attn"}
@@ -504,7 +529,7 @@ def main():
 
             def o_plain():
                 for L in L0: ext.q4_attn_2_tp(xa, ta, L.o.q4, True)
-            ga, gp = capture(o_ar), capture(o_plain)
+            ga, gp = capture(o_ar)[0], capture(o_plain)[0]
             for _ in range(2): ga.replay(); gp.replay()
             barrier(); ua = time_events(ga.replay, 8) * 1e3 / nl
             barrier(); up = time_events(gp.replay, 8) * 1e3 / nl

@@ -1,10 +1,31 @@
 """Shared helpers for the parity tests (test infrastructure; may import the oracle)."""
 import ctypes as C
+import functools
+import math
 import os
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_kernels.npz")
+
+
+def sample_idx(n, k=2048):
+    """k distinct flat indices spread over range(n) (all of them when n <= k): a fixed stride coprime with n, no RNG, so the
+    golden generator and the tests pick the same elements."""
+    if n <= k:
+        return np.arange(n)
+    p = 7919
+    while math.gcd(p, n) != 1:
+        p += 2
+    return np.sort((np.arange(k, dtype=np.int64) * p) % n)
+
+
+@functools.lru_cache(maxsize=None)
+def ref_golden():
+    """Outputs of the reference's own kernels on the tests' seeded inputs (oracle/gen_golden_ref_kernels.py)."""
+    return dict(np.load(REF_GOLDEN))
+
 
 # Stated fp16 tolerance for q4_matmul (SURVEY.md 8c): ours accumulates exact fp16 products in fp32, so the
 # only error against the float64 restatement is the final fp16 rounding (2^-11 relative) plus fp32 summation.

@@ -1,10 +1,10 @@
 """GPU parity of q4_matmul through the C ABI (ctypes -> libexl_b200.so), against the float64 oracle on the same
-seeded inputs, and -- when oracle/_ref/libexllama_ref.so travelled with the snapshot -- against the reference's
-own kernels compiled for sm_100a.  Tolerance: see helpers.REL_TOL / RMS_TOL (fp16 output rounding)."""
+seeded inputs, and against the outputs of the reference's own kernels compiled for sm_100a (tests/golden/ref_kernels.npz).
+Tolerance: see helpers.REL_TOL / RMS_TOL (fp16 output rounding)."""
 import numpy as np
 import pytest
 
-from helpers import RefLib, assert_close_ref64, to_cuda
+from helpers import assert_close_ref64, ref_golden, sample_idx, to_cuda
 
 pytestmark = pytest.mark.gpu
 
@@ -183,37 +183,39 @@ def test_reconstruct_bit_exact(oracle):
 
 
 # ---------------------------------------------------------------------------------------------------
-# against the reference's own kernels (oracle/_ref/libexllama_ref.so)
+# against the reference's own kernels (outputs stored by oracle/gen_golden_ref_kernels.py)
 # ---------------------------------------------------------------------------------------------------
 
-@pytest.fixture(scope="module")
-def reflib():
-    try:
-        r = RefLib()
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref/libexllama_ref.so not present")
-    r.prepare_buffers(inter=11008, max_rows=256, dq_numel=4096 * 11008)
-    return r
+REF_DECODE_CASES = [(1, 4096, 4096, 128, False), (1, 4096, 11008, 128, False), (4, 5120, 5120, 128, True), (7, 2048, 6656, 32, True)]
+REF_RECONS_CASE = (64, 4096, 4096, 128)
 
 
-@pytest.mark.parametrize("M,K,N,gs,act", [(1, 4096, 4096, 128, False), (1, 4096, 11008, 128, False),
-                                          (4, 5120, 5120, 128, True), (7, 2048, 6656, 32, True)])
-def test_against_reference_decode_kernel(oracle, reflib, M, K, N, gs, act):
+def ref_decode_inputs(oracle, M, K, N, gs, act):
+    return _mk(oracle, K, N, gs, act, seed=41) + (oracle.synth_x(M, K, seed=7),)
+
+
+def ref_recons_inputs(oracle):
+    M, K, N, gs = REF_RECONS_CASE
+    return _mk(oracle, K, N, gs, False, seed=43)[:3] + (oracle.synth_x(M, K, seed=8),)
+
+
+@pytest.mark.parametrize("M,K,N,gs,act", REF_DECODE_CASES)
+def test_against_reference_decode_kernel(oracle, M, K, N, gs, act):
     """|new - ref_ext| within 2e-2 (the reference accumulates in fp16 with atomics) AND our error against the
-    float64 restatement is no larger than the reference's own (SURVEY.md 8c)."""
-    import torch
+    float64 restatement is no larger than the reference's own (SURVEY.md 8c).  Compared at helpers.sample_idx positions."""
     from exllama_b200 import capi
-    qw, qz, sc, g_idx = _mk(oracle, K, N, gs, act, seed=41)
-    x = oracle.synth_x(M, K, seed=7)
-    mine = capi.q4_matmul(to_cuda(x), _q4(capi, qw, qz, sc, g_idx)).cpu().numpy().astype(np.float64)
-    tq, tz, ts = to_cuda(qw.copy(), qz, sc)
-    h = reflib.make_q4(tq, tz, ts, g_idx)
-    theirs = reflib.q4_matmul(to_cuda(x), h, N, mode=0).cpu().numpy().astype(np.float64)
+    qw, qz, sc, g_idx, x = ref_decode_inputs(oracle, M, K, N, gs, act)
+    g = ref_golden()
+    key = f"q4_decode_{M}_{K}_{N}_{gs}_{int(act)}"
+    idx = sample_idx(M * N)
+    mine = capi.q4_matmul(to_cuda(x), _q4(capi, qw, qz, sc, g_idx)).cpu().numpy().astype(np.float64).reshape(-1)[idx]
+    theirs = g[key].astype(np.float64)
     if act:
         # both implementations must have produced the same sequential qweight and x_map
-        np.testing.assert_array_equal(tq.cpu().numpy(), oracle.make_sequential(qw, oracle.make_x_map(g_idx, K // gs)))
+        seq = oracle.make_sequential(qw, oracle.make_x_map(g_idx, K // gs)).reshape(-1)
+        np.testing.assert_array_equal(g[key + "_qweight"], seq[sample_idx(seq.size)])
     # column sample for ref64 (full oracle is O(MKN) on the CPU)
-    ref_full = oracle.ref64_with_act_order(x, qw, qz, sc, g_idx) if K * N <= 4096 * 4096 * 2 else None
+    ref_full = oracle.ref64_with_act_order(x, qw, qz, sc, g_idx).reshape(-1)[idx] if K * N <= 4096 * 4096 * 2 else None
     rms = np.sqrt(np.mean(theirs ** 2))
     assert np.all(np.abs(mine - theirs) <= 2e-2 * np.abs(theirs) + 2e-2 * rms)
     if ref_full is not None:
@@ -221,14 +223,11 @@ def test_against_reference_decode_kernel(oracle, reflib, M, K, N, gs, act):
         assert e_mine <= e_ref * 1.05 + 1e-6, (e_mine, e_ref)
 
 
-def test_against_reference_recons_path(oracle, reflib):
+def test_against_reference_recons_path(oracle):
     from exllama_b200 import capi
-    M, K, N, gs = 64, 4096, 4096, 128
-    qw, qz, sc, _ = _mk(oracle, K, N, gs, False, seed=43)
-    x = oracle.synth_x(M, K, seed=8)
-    mine = capi.q4_matmul(to_cuda(x), _q4(capi, qw, qz, sc, None)).cpu().numpy().astype(np.float64)
-    tq, tz, ts = to_cuda(qw.copy(), qz, sc)
-    h = reflib.make_q4(tq, tz, ts, None)
-    theirs = reflib.q4_matmul(to_cuda(x), h, N, mode=1).cpu().numpy().astype(np.float64)
+    qw, qz, sc, x = ref_recons_inputs(oracle)
+    out = capi.q4_matmul(to_cuda(x), _q4(capi, qw, qz, sc, None)).cpu().numpy().astype(np.float64).reshape(-1)
+    mine = out[sample_idx(out.size)]
+    theirs = ref_golden()["q4_recons"].astype(np.float64)
     rms = np.sqrt(np.mean(theirs ** 2))
     assert np.all(np.abs(mine - theirs) <= 2e-2 * np.abs(theirs) + 2e-2 * rms)
