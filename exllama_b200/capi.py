@@ -60,6 +60,7 @@ SIGNATURES = {
     "exl_decode_plan_ipc_import": (i32, [vp, vp, i32]),
     "exl_launch_count": (i64, []),
     "exl_last_q4_path": (C.c_char_p, []),
+    "exl_last_tc_config": (C.c_char_p, []),
 }
 
 
@@ -214,6 +215,11 @@ def launch_count() -> int:
 
 def last_q4_path() -> str:
     return lib().exl_last_q4_path().decode()
+
+
+def last_tc_config() -> str:
+    """Tile configuration of the last tcgen05 GEMM launch ("128x128", "256x128", "256x256", "+mc" when multicast ran)."""
+    return lib().exl_last_tc_config().decode()
 
 
 class _DecodeDesc(C.Structure):

@@ -12,6 +12,7 @@
 ExlTuning g_tuning;
 std::atomic<int64_t> g_launches{0};
 const char* g_last_q4_path = "none";
+const char* g_last_tc_config = "none";
 
 static thread_local char t_err[1024] = "";
 static ExlDevice g_devices[EXL_MAX_DEVICES];
@@ -79,6 +80,7 @@ const char* exl_last_error(void) { return t_err; }
 int exl_version(void) { return 100; }
 int64_t exl_launch_count(void) { return g_launches.load(); }
 const char* exl_last_q4_path(void) { return g_last_q4_path; }
+const char* exl_last_tc_config(void) { return g_last_tc_config; }
 
 int exl_set_tuning_params(int matmul_recons_thd, int fused_mlp_thd, int sdp_thd, int matmul_fused_remap,
                           int rmsnorm_no_half2, int rope_no_half2, int matmul_no_half2, int silu_no_half2,

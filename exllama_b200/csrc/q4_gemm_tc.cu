@@ -428,6 +428,8 @@ int exl_tc_gemm_launch(ExlDevice* ds, const half* x, int M, const exl_q4_matrix*
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     lc.attrs = at; lc.numAttrs = mc ? 1 : 0;
+    static const char* const cfg_names[3][2] = {{"128x128", "128x128"}, {"256x128", "256x128+mc"}, {"256x256", "256x256+mc"}};
+    g_last_tc_config = cfg_names[cfg][mc];
     cudaError_t le = cudaLaunchKernelEx(&lc, kern, a);
     if (le != cudaSuccess) return exl_set_err(EXL_ERR_CUDA, "launch of q4_gemm_tc_kernel failed: %s", cudaGetErrorString(le));
     EXL_CHECK_LAUNCH("q4_gemm_tc_kernel");

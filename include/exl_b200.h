@@ -258,6 +258,9 @@ int exl_q4_matmul_host(const void* x_host, int M, const exl_q4_matrix* w, void* 
 int64_t exl_launch_count(void);
 /* name of the code path the last exl_q4_matmul call took ("skinny_mma", "tc_gemm", "recons_cublas") */
 const char* exl_last_q4_path(void);
+/* tile configuration of the last tcgen05 GEMM launch: "128x128", "256x128" or "256x256" (M x N per CTA), with the suffix
+   "+mc" when the x tile was multicast across a 2-CTA cluster; "none" before the first one */
+const char* exl_last_tc_config(void);
 
 #define EXL_SKINNY_MAX_M 8
 

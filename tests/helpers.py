@@ -124,3 +124,84 @@ class RefLib:
 
     def sync(self):
         self.lib.ref_sync()
+
+
+# ---------------------------------------------------------------------------------------------------
+# large GEMMs: float64 reference on a row / column sample
+# ---------------------------------------------------------------------------------------------------
+
+def tile_edge_sample(n, tile=128, edge=8):
+    """Sorted indices of range(n): the first and last `edge` of every full `tile`-sized block, and all of a partial last block
+    (where the tail handling of a tiled kernel lives)."""
+    full = n // tile
+    idx = [np.arange(b * tile, b * tile + edge) for b in range(full)] + [np.arange((b + 1) * tile - edge, (b + 1) * tile) for b in range(full)]
+    idx.append(np.arange(full * tile, n))
+    return np.unique(np.concatenate(idx)).astype(np.int64)
+
+
+def ref64_sampled(x, qw, qz, sc, g_idx, rows, cols, acc_in=None, recons=True):
+    """ref64_with_act_order(...)[rows][:, cols] without the full M x K x N contraction.  Both restrictions are exact: a row of the
+    product depends on that row of x only, a column on that column of the GPTQ tensors (and on g_idx, a property of K).
+    cols must be a multiple of 8 long (the zero points are repacked 8 per word)."""
+    from exllama_b200.tp import gather_q4_columns
+    from oracle import oracle as O
+    rows, cols = np.asarray(rows), np.asarray(cols)
+    xm = None
+    if g_idx is not None:
+        xm = O.make_x_map(g_idx, qz.shape[0])
+        qw = O.make_sequential(qw, xm)
+    sqw, sqz, ssc = gather_q4_columns(qw, qz, sc, cols)
+    acc = None if acc_in is None else np.ascontiguousarray(acc_in[rows][:, cols])
+    return O.q4_matmul_f64(np.ascontiguousarray(x[rows]), sqw, sqz, ssc, xm, acc, recons)
+
+
+# ---------------------------------------------------------------------------------------------------
+# decode step: synthetic stack and its float64 / fp16 oracle composition
+# ---------------------------------------------------------------------------------------------------
+
+def mk_stack(hidden, inter, layers, heads, gs, max_seq, vocab=2048, seed=3, act=False, with_head=True):
+    """Seeded synthetic GPTQ stack on cuda:0 with random (not zero) KV caches."""
+    import torch
+    from exllama_b200.stack import DecodeStack, LlamaShape
+    shape = LlamaShape("synthetic", hidden, inter, layers, heads, vocab=vocab)
+    st = DecodeStack(shape, groupsize=gs, act_order=act, device="cuda:0", max_seq=max_seq, seed=seed, with_head=with_head)
+    g = torch.Generator(device="cuda"); g.manual_seed(seed + 100)
+    for kc, vc in zip(st.key_cache, st.value_cache):
+        kc.copy_((torch.randn(kc.shape, device="cuda", generator=g) * 0.5).half())
+        vc.copy_((torch.randn(vc.shape, device="cuda", generator=g) * 0.5).half())
+    return st
+
+
+def oracle_step(oracle, st, x, past):
+    """float64/fp16 restatement of one decode token through the stack: returns (final hidden fp16, logits float64 or None without
+    lm_head, new k/v rows)."""
+    s = st.shape
+    hd, heads = s.head_dim, s.heads
+    sin = st.sin.view(-1, hd).cpu().numpy(); cos = st.cos.view(-1, hd).cpu().numpy()
+    x = x.reshape(1, s.hidden).copy()
+    rows = []
+
+    def mm(xin, lin, acc=None):
+        # make_q4 has already rewritten an act-order qweight into sequential order (q4_matrix.cu:159): contract with the x gather
+        xm = None if lin.g_idx is None else oracle.make_x_map(lin.g_idx.numpy(), lin.qzeros.shape[0])
+        return oracle.q4_matmul_f64(xin, lin.qweight.cpu().numpy(), lin.qzeros.cpu().numpy(), lin.scales.cpu().numpy(), xm, acc)
+    for i, L in enumerate(st.layers):
+        xn, _ = oracle.rms_norm(x, L.ln1.cpu().numpy(), s.eps)
+        q = mm(xn, L.q).astype(np.float16); k = mm(xn, L.k).astype(np.float16); v = mm(xn, L.v).astype(np.float16)
+        q = oracle.rope(q.reshape(1, heads, hd), sin, cos, 1, heads, hd, heads, past).reshape(-1)
+        k = oracle.rope(k.reshape(1, heads, hd), sin, cos, 1, heads, hd, heads, past).reshape(heads, hd)
+        kc = st.key_cache[i][0].cpu().numpy().copy(); vc = st.value_cache[i][0].cpu().numpy().copy()
+        kc[:, past] = k; vc[:, past] = v.reshape(heads, hd)
+        rows.append((k.copy(), v.reshape(heads, hd).copy()))
+        attn = oracle.decode_attn_f64(q, kc, vc, heads, heads, hd, past + 1, st.max_seq).astype(np.float16).reshape(1, -1)
+        x = mm(attn, L.o, acc=x).astype(np.float16)
+        xn, _ = oracle.rms_norm(x, L.ln2.cpu().numpy(), s.eps)
+        act = oracle.silu_mul(mm(xn, L.gate).astype(np.float16), mm(xn, L.up).astype(np.float16))
+        x = mm(act, L.down, acc=x).astype(np.float16)
+    if st.lm_head is None:
+        return x, None, rows
+    hn, _ = oracle.rms_norm(x, st.norm.cpu().numpy(), s.eps)
+    hn = hn.astype(np.float64).reshape(-1)
+    # in row blocks: a 32000 x 8192 head in float64 alone would be 2 GB of host memory
+    logits = np.concatenate([st.lm_head[r:r + 4096].cpu().numpy().astype(np.float64) @ hn for r in range(0, s.vocab, 4096)])
+    return x, logits.reshape(1, -1), rows

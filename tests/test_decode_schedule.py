@@ -87,12 +87,21 @@ def test_schedule_other_grids(lib, grid):
 
 
 def test_schedule_no_head_and_tiny(lib):
-    # the tiny shapes of tests/test_gpu_decode_step.py and __graft_entry__.smoke(); a plan without lm_head
-    for (H, I, heads, vocab) in [(1024, 2816, 8, 0), (1024, 2816, 8, 512), (512, 1536, 4, 256), (2048, 5632, 16, 32000)]:
+    # the tiny shapes of tests/test_gpu_decode_step.py, tests/test_gpu_decode_step_variants.py and __graft_entry__.smoke();
+    # a plan without lm_head; hidden = inter (one quantisation group per matrix); odd lm_head chunks per row (H 1536) with a
+    # vocabulary that leaves a partial last head stage (2052 * 3 % 8 != 0)
+    for (H, I, heads, vocab) in [(1024, 2816, 8, 0), (1024, 2816, 8, 512), (512, 1536, 4, 256), (2048, 5632, 16, 32000),
+                                 (1024, 2816, 8, 2048), (1024, 1024, 8, 2048), (2048, 2048, 16, 2048), (1536, 4096, 12, 2052),
+                                 (1536, 4096, 12, 2048)]:
         rc, msg = check(lib, H, heads * 128, I, heads, vocab, SMS, 0, 300, act=False)
         assert rc == 0, f"{(H, I, heads, vocab)}: {msg}"
         rc, msg = check(lib, H, heads * 128, I, heads, vocab, SMS, 0, 300, act=True)
         assert rc == 0, f"act {(H, I, heads, vocab)}: {msg}"
+    # the small shape on the grids the GPU tests set through EXL_DS_GRID, every context of its 256-position cache
+    for grid in (100, 132):
+        for act in (False, True):
+            rc, msg = check(lib, 1024, 1024, 2816, 8, 2048, grid, 0, 255, act=act)
+            assert rc == 0, f"grid {grid} act {act}: {msg}"
 
 
 def test_checker_rejects_bad_shapes(lib):

@@ -5,51 +5,9 @@ from the reference file:line the oracle cites -- and (b) this repo's own per-op 
 import numpy as np
 import pytest
 
-from helpers import assert_close_ref64
+from helpers import assert_close_ref64, mk_stack as _mk_stack, oracle_step as _oracle_step
 
 pytestmark = pytest.mark.gpu
-
-
-def _mk_stack(hidden, inter, layers, heads, gs, max_seq, vocab=2048, seed=3, act=False):
-    import torch
-    from exllama_b200.stack import DecodeStack, LlamaShape
-    shape = LlamaShape("synthetic", hidden, inter, layers, heads, vocab=vocab)
-    st = DecodeStack(shape, groupsize=gs, act_order=act, device="cuda:0", max_seq=max_seq, seed=seed)
-    g = torch.Generator(device="cuda"); g.manual_seed(seed + 100)
-    for kc, vc in zip(st.key_cache, st.value_cache):
-        kc.copy_((torch.randn(kc.shape, device="cuda", generator=g) * 0.5).half())
-        vc.copy_((torch.randn(vc.shape, device="cuda", generator=g) * 0.5).half())
-    return st
-
-
-def _oracle_step(oracle, st, x, past):
-    """float64/fp16 restatement of one decode token through the stack: returns (final hidden fp16, logits float64, new k/v rows)."""
-    s = st.shape
-    hd, heads = s.head_dim, s.heads
-    sin = st.sin.view(-1, hd).cpu().numpy(); cos = st.cos.view(-1, hd).cpu().numpy()
-    x = x.reshape(1, s.hidden).copy()
-    rows = []
-
-    def mm(xin, lin, acc=None):
-        # make_q4 has already rewritten an act-order qweight into sequential order (q4_matrix.cu:159): contract with the x gather
-        xm = None if lin.g_idx is None else oracle.make_x_map(lin.g_idx.numpy(), lin.qzeros.shape[0])
-        return oracle.q4_matmul_f64(xin, lin.qweight.cpu().numpy(), lin.qzeros.cpu().numpy(), lin.scales.cpu().numpy(), xm, acc)
-    for i, L in enumerate(st.layers):
-        xn, _ = oracle.rms_norm(x, L.ln1.cpu().numpy(), s.eps)
-        q = mm(xn, L.q).astype(np.float16); k = mm(xn, L.k).astype(np.float16); v = mm(xn, L.v).astype(np.float16)
-        q = oracle.rope(q.reshape(1, heads, hd), sin, cos, 1, heads, hd, heads, past).reshape(-1)
-        k = oracle.rope(k.reshape(1, heads, hd), sin, cos, 1, heads, hd, heads, past).reshape(heads, hd)
-        kc = st.key_cache[i][0].cpu().numpy().copy(); vc = st.value_cache[i][0].cpu().numpy().copy()
-        kc[:, past] = k; vc[:, past] = v.reshape(heads, hd)
-        rows.append((k.copy(), v.reshape(heads, hd).copy()))
-        attn = oracle.decode_attn_f64(q, kc, vc, heads, heads, hd, past + 1, st.max_seq).astype(np.float16).reshape(1, -1)
-        x = mm(attn, L.o, acc=x).astype(np.float16)
-        xn, _ = oracle.rms_norm(x, L.ln2.cpu().numpy(), s.eps)
-        act = oracle.silu_mul(mm(xn, L.gate).astype(np.float16), mm(xn, L.up).astype(np.float16))
-        x = mm(act, L.down, acc=x).astype(np.float16)
-    hn, _ = oracle.rms_norm(x, st.norm.cpu().numpy(), s.eps)
-    logits = hn.astype(np.float64) @ st.lm_head.cpu().numpy().astype(np.float64).T
-    return x, logits, rows
 
 
 @pytest.mark.parametrize("gs,act", [(128, False), (32, False), (256, False), (128, True), (32, True)])
