@@ -61,6 +61,7 @@ SIGNATURES = {
     "exl_launch_count": (i64, []),
     "exl_last_q4_path": (C.c_char_p, []),
     "exl_last_tc_config": (C.c_char_p, []),
+    "exl_last_gemv_config": (C.c_char_p, []),
 }
 
 
@@ -220,6 +221,12 @@ def last_q4_path() -> str:
 def last_tc_config() -> str:
     """Tile configuration of the last tcgen05 GEMM launch ("128x128", "256x128", "256x256", "+mc" when multicast ran)."""
     return lib().exl_last_tc_config().decode()
+
+
+def last_gemv_config() -> str:
+    """Decode GEMV launches of the last q4_* call, "; "-separated, each e.g. "rmsnorm+silu_mul cs=2 chunk=8 items=86"
+    (prologue+epilogue, cluster size = K split, x staging chunk in 128-k stages, clusters); "none" when it made none."""
+    return lib().exl_last_gemv_config().decode()
 
 
 class _DecodeDesc(C.Structure):

@@ -13,6 +13,7 @@ ExlTuning g_tuning;
 std::atomic<int64_t> g_launches{0};
 const char* g_last_q4_path = "none";
 const char* g_last_tc_config = "none";
+char g_last_gemv_config[512] = "";      // q4_gemv launches of the last exl_q4_* call (cleared on entry, appended by launch_cfg)
 
 static thread_local char t_err[1024] = "";
 static ExlDevice g_devices[EXL_MAX_DEVICES];
@@ -81,6 +82,7 @@ int exl_version(void) { return 100; }
 int64_t exl_launch_count(void) { return g_launches.load(); }
 const char* exl_last_q4_path(void) { return g_last_q4_path; }
 const char* exl_last_tc_config(void) { return g_last_tc_config; }
+const char* exl_last_gemv_config(void) { return g_last_gemv_config[0] ? g_last_gemv_config : "none"; }
 
 int exl_set_tuning_params(int matmul_recons_thd, int fused_mlp_thd, int sdp_thd, int matmul_fused_remap,
                           int rmsnorm_no_half2, int rope_no_half2, int matmul_no_half2, int silu_no_half2,
@@ -264,6 +266,7 @@ static int q4_matmul_dispatch(ExlDevice* ds, const half* x, int M, const exl_q4_
 
 int exl_q4_matmul(const void* x, int M, const exl_q4_matrix* w, void* out, int no_zero, int force_path, void* stream)
 {
+    g_last_gemv_config[0] = 0;
     if (!w) return exl_set_err(EXL_ERR_STATE, "q4_matmul: NULL handle");
     ExlDevice* ds = exl_device_state(w->device);
     if (!ds) return EXL_ERR_CUDA;
@@ -282,6 +285,7 @@ int exl_q4_reconstruct(const exl_q4_matrix* w, void* out, void* stream)
 int exl_q4_matmul_lora(const void* x, int M, const exl_q4_matrix* w, void* out, const void* lora_A, const void* lora_B,
                        int rank, void* lora_temp, void* stream_)
 {
+    g_last_gemv_config[0] = 0;
     if (!w) return exl_set_err(EXL_ERR_STATE, "q4_matmul_lora: NULL handle");
     ExlDevice* ds = exl_device_state(w->device);
     if (!ds) return EXL_ERR_CUDA;
@@ -349,6 +353,7 @@ int exl_q4_attn(void* x_, const void* rms_norm_weight, float epsilon, void* quer
                 const void* q_a, const void* q_b, int q_rank, const void* k_a, const void* k_b, int k_rank,
                 const void* v_a, const void* v_b, int v_rank, void* lora_temp, int device, void* stream_)
 {
+    g_last_gemv_config[0] = 0;
     if (!q_proj || !k_proj || !v_proj) return exl_set_err(EXL_ERR_STATE, "q4_attn: NULL handle");
     ExlDevice* ds = exl_device_state(device);
     if (!ds) return EXL_ERR_CUDA;
@@ -408,6 +413,7 @@ int exl_q4_attn(void* x_, const void* rms_norm_weight, float epsilon, void* quer
 int exl_q4_attn_2(void* x, const void* attn_output, const exl_q4_matrix* o_proj, int height,
                   const void* o_a, const void* o_b, int o_rank, void* lora_temp, void* stream_)
 {
+    g_last_gemv_config[0] = 0;
     if (!o_proj) return exl_set_err(EXL_ERR_STATE, "q4_attn_2: NULL handle");
     ExlDevice* ds = exl_device_state(o_proj->device);
     if (!ds) return EXL_ERR_CUDA;
@@ -427,6 +433,7 @@ static int q4_mlp_impl(void* x_, const void* rms_norm_weight, float epsilon, con
                const void* up_a, const void* up_b, int up_rank, const void* down_a, const void* down_b, int down_rank,
                void* lora_temp, int device, void* stream_, bool add_residual, bool all_reduce = false)
 {
+    g_last_gemv_config[0] = 0;
     if (!gate || !up || !down) return exl_set_err(EXL_ERR_STATE, "q4_mlp: NULL handle");
     ExlDevice* ds = exl_device_state(device);
     if (!ds) return EXL_ERR_CUDA;
@@ -506,6 +513,7 @@ int exl_q4_mlp_ar(void* x, const void* rms_norm_weight, float epsilon, const exl
 
 int exl_q4_attn_2_ar(void* x, const void* attn_output, const exl_q4_matrix* o_proj, int height, void* stream)
 {
+    g_last_gemv_config[0] = 0;
     if (!o_proj) return exl_set_err(EXL_ERR_STATE, "q4_attn_2_ar: NULL handle");
     ExlDevice* ds = exl_device_state(o_proj->device);
     if (!ds) return EXL_ERR_CUDA;
@@ -566,6 +574,7 @@ int exl_tp_status(int device, unsigned* timeouts)
 
 int exl_q4_attn_2_tp(void* x, const void* attn_output, const exl_q4_matrix* o_proj, int height, int add_residual, void* stream)
 {
+    g_last_gemv_config[0] = 0;
     if (!o_proj) return exl_set_err(EXL_ERR_STATE, "q4_attn_2_tp: NULL handle");
     ExlDevice* ds = exl_device_state(o_proj->device);
     if (!ds) return EXL_ERR_CUDA;
@@ -582,6 +591,7 @@ int exl_decode_attn(const void* q, const void* key_cache, const void* value_cach
 
 int exl_q4_matmul_host(const void* x_host, int M, const exl_q4_matrix* w, void* out_host, void* d_x, void* d_out, void* stream_)
 {
+    g_last_gemv_config[0] = 0;
     if (!w) return exl_set_err(EXL_ERR_STATE, "q4_matmul_host: NULL handle");
     ExlDevice* ds = exl_device_state(w->device);
     if (!ds) return EXL_ERR_CUDA;

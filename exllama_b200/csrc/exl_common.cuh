@@ -87,6 +87,7 @@ extern ExlTuning g_tuning;
 extern std::atomic<int64_t> g_launches;
 extern const char* g_last_q4_path;
 extern const char* g_last_tc_config;
+extern char g_last_gemv_config[512];
 
 enum ExlScratchRole { SCR_NORM = 0, SCR_MLP = 1, SCR_DQ = 2, SCR_REMAP = 3 };
 int exl_own_scratch(ExlDevice* ds, int role, int64_t numel, half** out);   // grow-only, lazy; not CUDA-graph safe on first use

@@ -870,6 +870,11 @@ int launch_cfg(ExlDevice* ds, GemvArgs& a, int items, cudaStream_t stream)
     if (force_cs >= 1 && force_cs <= MAX_CS && force_cs <= a.spt && nsub * force_cs * a.M * GV_TILE_N * (int)sizeof(float) <= SLOT_BUDGET) cs = force_cs;
     a.cs = cs;
     const size_t smem = smem_for(cs);
+    static const char* const pro_names[2] = {"plain", "rmsnorm"};
+    static const char* const epi_names[4] = {"store", "silu_mul", "rope_cache", "allreduce"};
+    const size_t used = strlen(g_last_gemv_config);       // one entry per launch of the current exl_q4_* call, in launch order
+    snprintf(g_last_gemv_config + used, sizeof(g_last_gemv_config) - used, "%s%s+%s cs=%d chunk=%d items=%d", used ? "; " : "",
+             pro_names[PRO], epi_names[EPI], cs, a.chunk_stages, items);
 
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));

@@ -261,6 +261,10 @@ const char* exl_last_q4_path(void);
 /* tile configuration of the last tcgen05 GEMM launch: "128x128", "256x128" or "256x256" (M x N per CTA), with the suffix
    "+mc" when the x tile was multicast across a 2-CTA cluster; "none" before the first one */
 const char* exl_last_tc_config(void);
+/* decode GEMV (q4_gemv_kernel) launches of the last exl_q4_* call, in launch order and separated by "; ", each
+   "<prologue>+<epilogue> cs=<cluster size = K split> chunk=<x staging chunk, 128-k stages> items=<clusters>", e.g.
+   "rmsnorm+silu_mul cs=2 chunk=8 items=86; plain+store cs=4 chunk=8 items=32" for a fused q4_mlp; "none" when it made none */
+const char* exl_last_gemv_config(void);
 
 #define EXL_SKINNY_MAX_M 8
 

@@ -12,28 +12,11 @@ import numpy as np
 import pytest
 
 from helpers import assert_close_ref64, mk_stack, oracle_step
+from helpers import sharper as _sharper
 
 pytestmark = pytest.mark.gpu
 
 SMALL = (1024, 2816, 8)          # hidden, inter, heads of the small test shape
-
-
-def _rms(a):
-    return float(np.sqrt(np.mean(np.square(np.asarray(a, dtype=np.float64)))))
-
-
-def _sharper(fused, per_op, want, what):
-    """fused-vs-oracle rms error <= 1.25 x per-op-vs-oracle rms error + 1e-4 x rms; returns the ratio of the two errors.
-    The new K / V rows are one fp16 rounding from the oracle on both paths (errors ~1e-4 of rms), where single-ulp rounding
-    flips alone move the ratio up to ~1.5 (measured on a B200, median 0.98 over all cases): the 1e-4 x rms term covers that."""
-    want = np.asarray(want, dtype=np.float64).reshape(-1)
-    e_f = _rms(np.asarray(fused, dtype=np.float64).reshape(-1) - want)
-    e_p = _rms(np.asarray(per_op, dtype=np.float64).reshape(-1) - want)
-    r = _rms(want)
-    assert e_f <= 1.25 * e_p + 1e-4 * r, f"{what}: fused rms err {e_f:.4g} vs per-op {e_p:.4g} (rms {r:.4g})"
-    ratio = e_f / max(e_p, 1e-30)
-    print(f"{what}: fused/per-op rms error ratio {ratio:.3f} (fused {e_f / r:.3e}, per-op {e_p / r:.3e} of rms)")
-    return ratio
 
 
 def _restore(st, snap):
